@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...        (the reference's CPU path: the oracle port, host cores)
+    python bench.py ... --dump-outputs DIR      (also writes the last timed step's occupancy volume, see dump_volume)
 
 A "step" = one pass of the hot path over one synthetic frame: upload-free channel-last repack of the [1,256,128,128]
 feature map + the fused sample+MLP kernel over the dense 257^3 node grid ("256^3", RTL/main.py:187), z-slab
@@ -33,6 +34,7 @@ FLOP_PER_POINT = 2363906          # 2*(257*1024+1281*512+769*256+513*128+385*1) 
 # bench run: profiling and timing never share a run).  Updated by hand from profiles/ when the kernel changes.
 TRAFFIC_NCU = {"bytes": 82.69e6, "source": "profiles/r02_final_ncu_tc_summary.txt: 44.79 MB read + 37.90 MB written (ncu --set full pass of tools/gpu_r02_final.sh)"}
 B_MIN, B_MAX = (-1.0, -1.0, -1.0), (1.0, 1.0, 1.0)
+DUMP_NODES = 1 << 22              # --dump-outputs: a volume with more nodes is sampled (16 MB of values + 32 MB of node ids)
 
 
 def parse():
@@ -50,7 +52,12 @@ def parse():
     ap.add_argument("--fused-gather", action="store_true", help="same as --exchange fused")
     ap.add_argument("--no-recon", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the occupancy volume of the last timed step as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
+    return a
 
 
 def peaks():
@@ -156,6 +163,22 @@ def scene_calib():
     return pifu_calib(E, K, device="cpu")
 
 
+def dump_volume(dirname, vol):
+    """--dump-outputs: the volume as `volume.npy` (float32, z-major [R,R,R]) when it has at most DUMP_NODES nodes, else a fixed
+    seeded sample of DUMP_NODES nodes as `volume_sample.npy` (float32) with their linear z-major node ids in
+    `volume_sample_node.npy` (float64), so that two builds can be compared value for value."""
+    import numpy as np
+    import torch
+    if vol.numel() <= DUMP_NODES:
+        arrays = {"volume": vol}
+    else:
+        node = torch.randint(0, vol.numel(), (DUMP_NODES,), generator=torch.Generator().manual_seed(29))
+        arrays = {"volume_sample": vol.reshape(-1)[node.to(vol.device)], "volume_sample_node": node.double()}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------------------
 def best_threads(fn):
     """The torch-CPU port does not scale to every hardware thread of a big host: time a small sample at a few thread
@@ -193,10 +216,12 @@ def run_reference(args):
     times = []
     for i in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        spec.query_ref(feats[0], pts, cal, Ws, bs, spec.LAST_SIGMOID)
+        occ = spec.query_ref(feats[0], pts, cal, Ws, bs, spec.LAST_SIGMOID)
         dt = time.perf_counter() - t0
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_volume(args.dump_outputs, occ.reshape(S, S, S))
     total = sum(times)
     mpts = S ** 3 * len(times) / total / 1e6
     line = {
@@ -307,6 +332,8 @@ def run_ours(args):
         ev[i][1].record()
     barrier()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_volume(args.dump_outputs, vol)
     t_ms = sum(a.elapsed_time(b) for a, b in ev)
     k_ms = sum(a.elapsed_time(b) for a, b in kev)
     tt = torch.tensor([t_ms, k_ms], dtype=torch.float64, device=dev)

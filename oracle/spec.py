@@ -53,6 +53,30 @@ def make_points(N, seed, lo=-1.1, hi=1.1):
     return (torch.rand(1, 3, N, generator=g) * (hi - lo) + lo).contiguous()
 
 
+def make_encoder_state(layout, seed):
+    """float64 parameters for a state-dict layout [(key, shape), ...], drawn in layout order from one generator: weights
+    of rank > 1 U(-1/sqrt(fan_in), +1/sqrt(fan_in)) like the conv default init, norm scales 1 + U(-1/4, 1/4), biases
+    U(-1/4, 1/4)."""
+    g = torch.Generator().manual_seed(int(seed))
+    sd = {}
+    for key, shape in layout:
+        t = torch.rand(tuple(shape), generator=g, dtype=torch.float64) * 2 - 1
+        if len(shape) > 1:
+            t = t / math.sqrt(math.prod(shape[1:]))
+        elif key.endswith(".weight"):
+            t = 1 + 0.25 * t
+        else:
+            t = 0.25 * t
+        sd[key] = t
+    return sd
+
+
+def make_image(size, seed):
+    """[1,3,size,size] float64 image in [-1,1) (the encoders' input range)."""
+    g = torch.Generator().manual_seed(int(seed))
+    return torch.rand(1, 3, size, size, generator=g, dtype=torch.float64) * 2 - 1
+
+
 def _rot(rx, ry, rz):
     """Rotation R = Rz * Ry * Rx (RTL/scene.py:62-88 make_rotate)."""
     sx, cx, sy, cy, sz, cz = math.sin(rx), math.cos(rx), math.sin(ry), math.cos(ry), math.sin(rz), math.cos(rz)

@@ -10,6 +10,7 @@ are NOT stored: they are regenerated from seeds by oracle.spec.make_weights/make
 generator -- bit-reproducible for the pinned torch build); each file stores float64 checksums of the
 regenerated tensors so RNG drift is detected instead of silently failing parity.
 """
+import json
 import os
 import sys
 
@@ -139,10 +140,71 @@ def gen_calib(ns):
                         calib=np.stack([r["calib"] for r in rows]))
 
 
+@torch.no_grad()
+def gen_query_pitch70(ns):
+    """One more netG case at a steep camera pitch (yaw 20, pitch -70) on a 64x64 map, as the reference's query() returns it
+    for a single-stage feature list; the inputs are regenerated from their seeds and pinned by checksums."""
+    net = ns.PIFuNetG().eval()
+    Ws, bs = spec.make_weights(spec.G_CHANNELS, 5)
+    load_head(net, Ws, bs)
+    feat = spec.make_feat(256, 64, 64, 6)
+    pts = spec.make_points(3000, 7)
+    ref = net.query([[feat]], pts, calibs=spec.scene_calib(20, -70))[0][0]
+    np.savez_compressed(os.path.join(HERE, "reference_query_pitch70.npz"), expected=ref.numpy(),
+                        w_checksum=np.stack([checksum(w) for w in Ws]), f_checksum=checksum(feat), p_checksum=checksum(pts))
+
+
+ENCODER_SEED, ENCODER_IMAGE_SEED, ENCODER_IMAGE_SIZE, ENCODER_SAMPLE = 91, 92, 64, 1024
+
+
+@torch.no_grad()
+def gen_encoders(ns):
+    """Image encoders of PIFuNetG (HGFilter) and PIFuNetC (ResnetFilter) in float64 with seeded parameters: the state-dict
+    layout, checksums of the parameters as loaded (aliased keys keep the value loaded last), and of every stage's output a
+    checksum plus a seeded sample of ENCODER_SAMPLE values (whole outputs would be 1 MB)."""
+    rec = dict(seed=ENCODER_SEED, image_seed=ENCODER_IMAGE_SEED, image_size=ENCODER_IMAGE_SIZE)
+    for net, factory in (("G", ns.PIFuNetG), ("C", ns.PIFuNetC)):
+        ref = factory().eval().double()
+        layout = [(k, list(v.shape)) for k, v in ref.state_dict().items()]
+        ref.load_state_dict(spec.make_encoder_state(layout, ENCODER_SEED), strict=True)
+        outs = [o[0] for o in ref.image_filter(spec.make_image(ENCODER_IMAGE_SIZE, ENCODER_IMAGE_SEED))]
+        idx = torch.randint(0, outs[0].numel(), (ENCODER_SAMPLE,), generator=torch.Generator().manual_seed(ENCODER_SEED))
+        rec[net + "_layout"] = np.array(json.dumps(layout))
+        rec[net + "_state_checksum"] = np.stack([checksum(v) for v in ref.state_dict().values()])
+        rec[net + "_out_checksum"] = np.stack([checksum(o) for o in outs])
+        rec[net + "_out_index"] = idx.numpy()
+        rec[net + "_out_sample"] = np.stack([o.reshape(-1)[idx].numpy() for o in outs])
+        print("encoder %s: %d state entries, %d stage outputs of %s" % (net, len(layout), len(outs), tuple(outs[0].shape)))
+    np.savez_compressed(os.path.join(HERE, "encoders.npz"), **rec)
+
+
+def gen_obj_writer():
+    """Bytes of the reference's text OBJ writers (monoport/lib/mesh_util.py:223-242) for a small seeded mesh."""
+    import importlib.util
+    import tempfile
+    from oracle.ref_loader import REF_ROOT
+    spec_ = importlib.util.spec_from_file_location("_ref_mesh_util", os.path.join(REF_ROOT, "monoport", "lib", "mesh_util.py"))
+    ref = importlib.util.module_from_spec(spec_)
+    spec_.loader.exec_module(ref)
+    rng = np.random.default_rng(0)
+    V = rng.normal(size=(57, 3)).astype(np.float32)
+    F = rng.integers(0, 57, size=(101, 3)).astype(np.int32)
+    C = rng.random((57, 3)).astype(np.float32)
+    with tempfile.TemporaryDirectory() as d:
+        a, b = os.path.join(d, "a.obj"), os.path.join(d, "b.obj")
+        ref.save_obj_mesh(a, V, F)
+        ref.save_obj_mesh_with_color(b, V, F, C)
+        obj, obj_color = open(a).read(), open(b).read()
+    np.savez_compressed(os.path.join(HERE, "obj_writer.npz"), V=V, F=F, C=C, obj=np.array(obj), obj_color=np.array(obj_color))
+
+
 if __name__ == "__main__":
     torch.set_num_threads(8)
     ns = load_reference()
     gen_query(ns)
     gen_forward_vertices(ns)
     gen_calib(ns)
+    gen_query_pitch70(ns)
+    gen_encoders(ns)
+    gen_obj_writer()
     print("done")

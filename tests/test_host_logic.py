@@ -1,11 +1,13 @@
 """CPU: host-side logic -- drop-in import surface, encoder/state-dict compatibility, slab partition, MC table and
 octree oracle properties."""
+import json
 import os
 import numpy as np
 import pytest
 import torch
 
 from oracle import spec
+from helpers import GOLDEN, checksum
 
 
 def test_dropin_import_surface():
@@ -26,21 +28,30 @@ def test_dropin_import_surface():
 
 
 def test_encoders_match_reference_if_present():
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("reference tree not present (GPU box)")
-    ns = ref_loader.load_reference()
+    """For netG and netC: the reference's state dict loads strictly (same keys and shapes, aliased keys resolve to the same
+    values) and the image encoder returns the reference's stage outputs (tests/golden/encoders.npz, written by
+    make_golden.py from the reference).  The run is in float64 so that the stored outputs hold on any CPU: the bound is
+    summation-order noise, far below any difference in what is computed."""
+    g = np.load(os.path.join(GOLDEN, "encoders.npz"))
+    for net in ("G", "C"):
+        _check_encoder_against_golden(g, net)
+
+
+def _check_encoder_against_golden(g, net):
     from monoport_b200.modeling import PIFuNetG, PIFuNetC
-    torch.manual_seed(0)
-    for mk, rk in ((PIFuNetG, ns.PIFuNetG), (PIFuNetC, ns.PIFuNetC)):
-        mine, ref = mk().eval(), rk().eval()
-        mine.load_state_dict(ref.state_dict(), strict=True)
-        img = torch.randn(1, 3, 64, 64)
-        with torch.no_grad():
-            a, b = ref.image_filter(img), mine.image_filter(img)
-        assert len(a) == len(b)
-        for x, y in zip(a, b):
-            assert torch.equal(x[0], y[0])
+    layout = json.loads(str(g[net + "_layout"]))
+    mine = (PIFuNetG if net == "G" else PIFuNetC)().eval().double()
+    mine.load_state_dict(spec.make_encoder_state(layout, int(g["seed"])), strict=True)
+    loaded = mine.state_dict()
+    np.testing.assert_allclose(np.stack([checksum(loaded[k]) for k, _ in layout]), g[net + "_state_checksum"], rtol=1e-12, atol=0)
+    with torch.no_grad():
+        outs = [o[0] for o in mine.image_filter(spec.make_image(int(g["image_size"]), int(g["image_seed"])))]
+    assert len(outs) == len(g[net + "_out_checksum"])
+    idx = torch.from_numpy(g[net + "_out_index"])
+    for o, want_sum, want_sample in zip(outs, g[net + "_out_checksum"], g[net + "_out_sample"]):
+        assert o.dtype == torch.float64
+        np.testing.assert_allclose(o.reshape(-1)[idx].numpy(), want_sample, rtol=1e-11, atol=1e-11)
+        np.testing.assert_allclose(checksum(o), want_sum, rtol=1e-11, atol=1e-11)
 
 
 def test_geometry_helpers_match_oracle():
@@ -136,39 +147,30 @@ def test_level_points_convention():
 
 
 def test_obj_writer_matches_reference_format(tmp_path):
-    """Same bytes as monoport/lib/mesh_util.py:223-242 (run against the reference when it is present)."""
+    """Same bytes as monoport/lib/mesh_util.py:223-242 writes (tests/golden/obj_writer.npz)."""
     from monoport.lib.mesh_util import save_obj_mesh, save_obj_mesh_with_color
-    rng = np.random.default_rng(0)
-    V = rng.normal(size=(57, 3)).astype(np.float32)
-    Fc = rng.integers(0, 57, size=(101, 3)).astype(np.int32)
-    C = rng.random((57, 3)).astype(np.float32)
+    g = np.load(os.path.join(GOLDEN, "obj_writer.npz"))
+    V, Fc, C = g["V"], g["F"], g["C"]
     a, b = tmp_path / "a.obj", tmp_path / "b.obj"
     save_obj_mesh(str(a), V, Fc)
     save_obj_mesh_with_color(str(b), torch.from_numpy(V), torch.from_numpy(Fc), C)
     la, lb = a.read_text().splitlines(), b.read_text().splitlines()
     assert len(la) == 57 + 101 and la[0] == "v %.4f %.4f %.4f" % tuple(V[0]) and la[57] == "f %d %d %d" % tuple(Fc[0] + 1)
     assert lb[0] == "v %.4f %.4f %.4f %.4f %.4f %.4f" % (tuple(V[0]) + tuple(C[0]))
-    from oracle import ref_loader
-    if ref_loader.available():
-        import importlib.util, os
-        spec_ = importlib.util.spec_from_file_location("_ref_mesh_util", os.path.join(ref_loader.REF_ROOT, "monoport/lib/mesh_util.py"))
-        ref = importlib.util.module_from_spec(spec_)
-        spec_.loader.exec_module(ref)
-        ra, rb = tmp_path / "ra.obj", tmp_path / "rb.obj"
-        ref.save_obj_mesh(str(ra), V, Fc)
-        ref.save_obj_mesh_with_color(str(rb), V, Fc, C)
-        assert ra.read_text() == a.read_text() and rb.read_text() == b.read_text()
+    assert a.read_text() == str(g["obj"]) and b.read_text() == str(g["obj_color"])
 
 
-def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` (the oracle port on the host cores) prints ONE JSON line with the contract's keys."""
+def test_bench_reference_arm_contract(tmp_path):
+    """`bench.py --impl reference` (the oracle port on the host cores) prints ONE JSON line with the contract's keys, and
+    `--dump-outputs` writes the volume its timed step computed."""
     import json
     import os
     import subprocess
     import sys
     from conftest import ROOT
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
-                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    out = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -180,6 +182,15 @@ def test_bench_reference_arm_contract():
     assert d["value"] > 0 and d["higher_is_better"] is True and d["vs_baseline"] is None and "workload" in d["config"]
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"]["value"] == d["value"] and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+    assert d["steps"] == 1 and sorted(os.listdir(out)) == ["volume.npy"]
+    import bench
+    _, Ws, bs, feats = bench.synthetic()
+    S = 48
+    pts = spec.level_points(spec._grid_coords(S, 1), S, bench.B_MIN, bench.B_MAX).t().contiguous()
+    want = spec.query_ref(feats[0], pts, bench.scene_calib(), Ws, bs, spec.LAST_SIGMOID).reshape(S, S, S)
+    vol = np.load(out / "volume.npy")
+    assert vol.dtype == np.float32
+    np.testing.assert_allclose(vol, want.numpy(), rtol=0, atol=1e-6)      # the bench may run on another thread count
 
 
 def test_binary_ply_round_trip(tmp_path):

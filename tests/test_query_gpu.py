@@ -393,3 +393,34 @@ def test_bench_head_tensor_core_vs_oracle():
         net.precision = mode
         got = net.query([[feats[0].cuda()]], world[None].cuda(), calibs=cal.cuda())[0][0, 0].cpu()
         assert (got - want).abs().max().item() <= TOL[mode], (mode, (got - want).abs().max().item())
+
+
+def test_bench_dump_outputs_is_the_last_timed_volume(tmp_path):
+    """`bench.py --dump-outputs`: the sampled volume it writes is the volume of its last timed step (feature map
+    (steps - 1) % 4), bit for bit, at the node ids written beside it; the line reports the number of timed steps asked for."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import bench
+    from conftest import ROOT
+    out = tmp_path / "out"
+    steps = 3
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--mode", "auto",
+                        "--no-recon", "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True,
+                       timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps
+    assert sorted(os.listdir(out)) == ["volume_sample.npy", "volume_sample_node.npy"]
+    sample, node = np.load(out / "volume_sample.npy"), np.load(out / "volume_sample_node.npy")
+    assert sample.dtype == np.float32 and node.dtype == np.float64 and sample.shape == node.shape == (bench.DUMP_NODES,)
+    _, Ws, bs, feats = bench.synthetic(n_feat=4)
+    net = build_net("G", Ws, bs)
+    net.precision = "auto"
+    R = bench.R_GRID
+    vol = net.query_grid(feats[(steps - 1) % len(feats)].cuda(), bench.scene_calib(), R, bench.B_MIN, bench.B_MAX)
+    got = vol.reshape(-1)[torch.from_numpy(node).long().cuda()].cpu()
+    assert torch.equal(got, torch.from_numpy(sample))
+    other = net.query_grid(feats[steps % len(feats)].cuda(), bench.scene_calib(), R, bench.B_MIN, bench.B_MAX)
+    assert not torch.equal(other.reshape(-1)[torch.from_numpy(node).long().cuda()].cpu(), got), "the frames must differ"
